@@ -5,9 +5,10 @@
   python -m torch.distributed.run --nnodes=1 --nproc-per-node N --master-addr 127.0.0.1 --master-port P \
          bench.py --gpus N --steps K --warmup W                     # N ranks, NCCL, weak scaling (32 images / GPU)
   python bench.py --impl reference --steps 3 --warmup 1             # the reference's CPU path (oracle port) on host cores
+  python bench.py --steps 20 --warmup 3 --dump-outputs DIR          # also write the last timed step's detections to DIR
 
 Workload (BASELINE.json configs[1]): SSD300, batch 32 synthetic 300x300x3 float32 images, 21 classes, 8732 priors,
-he_normal random weights, DecodeDetections(conf 0.01, iou 0.45, top_k 200, nms cap 400).
+he_normal random weights (conv1_1 scaled by 1/64, see _weights), DecodeDetections(conf 0.01, iou 0.45, top_k 200, nms cap 400).
 A step = one forward + decode of one batch.  `value` = images/s with inputs resident in HBM (CUDA events, max over
 ranks); `e2e` = the same through SSDModel.predict with pinned host images copied H2D and the (B,200,6) result copied
 D2H inside the timed region.
@@ -29,7 +30,7 @@ BATCH = 32
 N_CLASSES = 20
 METRIC = 'SSD300 images/sec (fwd+decode)'
 WORKLOAD = ('SSD300 inference, batch 32 per GPU, synthetic 300x300x3 float32, 21 classes, 8732 priors, he_normal random '
-            'weights, DecodeDetections(0.01/0.45/200/400)')
+            'weights (conv1_1 scaled by 1/64), DecodeDetections(0.01/0.45/200/400)')
 
 
 def _peaks():
@@ -42,9 +43,15 @@ def _peaks():
 
 
 def _weights():
+    """he_normal weights, zero biases, conv1_1 scaled by 1/64.  With zero biases the ReLU network is linear in the scale of its
+    input, and the default preprocessing leaves pixels within +-128: unscaled, the box regressions of the heads after conv4_3
+    reach ~1000, exp() overflows float32 in the decoder (infinite box coordinates) and every score saturates to 1.0.  The
+    scaled first layer keeps activations in the O(1) range that trained weights produce, so the detections are finite and
+    ranked by distinct scores."""
     from oracle import synth
     from oracle.model import vgg_weight_shapes
     w = synth.synth_weights(1, vgg_weight_shapes(300, N_CLASSES), bias_scale=0.0)
+    w['conv1_1/kernel'] = w['conv1_1/kernel'] / np.float32(64.0)
     w['conv4_3_norm/gamma'] = np.full((512,), 20.0, np.float32)
     return w
 
@@ -106,7 +113,7 @@ def _decode_one(y):
     C++ in TensorFlow -- runs through the C restatement oracle/tf_nms.c (bit-identical to the NumPy one, which stays the fallback
     where no compiler exists): a Python NMS loop would make the CPU arm slower than the reference really is."""
     from oracle.decoder import decode_layer, tf_nms_c
-    with np.errstate(all='ignore'):                 # random weights produce inf/NaN boxes (handled as TensorFlow does)
+    with np.errstate(all='ignore'):                 # overflowing boxes, should other weights produce them, are handled as TensorFlow does
         return decode_layer(y, 0.01, 0.45, 200, 400, True, 300, 300, nms=tf_nms_c)
 
 
@@ -291,6 +298,14 @@ def micro_benchmarks(peaks):
     out['train_step_ssd300_b32'] = {'ms': ms, 'images_per_s': Bt * 1e3 / ms, 'algorithmic_TFLOPs': fl / ms / 1e9,
                                     'frac_tensor_peak': fl / ms / 1e9 / peaks['bf16_tflops_sustained'], 'n_params': tr.n_params}
     return out
+
+
+def dump_outputs(path, arrays):
+    """Writes every array as `path/<name>.npy` in float32, so that two builds can be compared output for output (the inputs
+    and weights are seeded: the same arguments give the same inputs)."""
+    os.makedirs(path, exist_ok=True)
+    for name, a in arrays.items():
+        np.save(os.path.join(path, name + '.npy'), np.ascontiguousarray(a, dtype=np.float32))
 
 
 def _max_over_ranks(ms, dist):
@@ -487,6 +502,7 @@ def run_ours(args):
         torch.cuda.synchronize()
 
     def timed(fn, steps, warmup):
+        """Returns the time of `steps` calls, the clocks, the launch count and what the last call returned."""
         for i in range(warmup):
             fn(i)
         barrier()
@@ -495,8 +511,9 @@ def run_ours(args):
         l0 = _ffi.launch_count()
         e0, e1 = torch.cuda.Event(enable_timing=True), torch.cuda.Event(enable_timing=True)
         e0.record()
+        out = None
         for i in range(steps):
-            fn(warmup + i)
+            out = fn(warmup + i)
         e1.record()
         barrier()
         ms = e0.elapsed_time(e1)
@@ -505,9 +522,11 @@ def run_ours(args):
         if world > 1:
             t = torch.tensor([ms], device='cuda'); dist.all_reduce(t, op=dist.ReduceOp.MAX); ms = float(t.item())
             c = torch.tensor([launches], device='cuda', dtype=torch.int64); dist.all_reduce(c); launches = int(c.item())
-        return ms, clocks, launches
+        return ms, clocks, launches, out
 
-    ms_dev, clocks, launches = timed(step_device, args.steps, max(args.warmup, 3))
+    ms_dev, clocks, launches, last = timed(step_device, args.steps, max(args.warmup, 3))
+    if args.dump_outputs and rank == 0:
+        dump_outputs(args.dump_outputs, {'detections': last.cpu().numpy()})
     # end to end: one untimed pipelined pass, then K batches in ONE timed pipelined pass (K uploads + K downloads inside it)
     run_e2e(max(args.warmup, 3))
     barrier()
@@ -622,7 +641,13 @@ def main():
     ap.add_argument('--fast', action='store_true', help='single-pass bf16 convolutions instead of bf16x3')
     ap.add_argument('--no-cpu', action='store_true')
     ap.add_argument('--no-micro', action='store_true')
+    ap.add_argument('--dump-outputs', metavar='DIR',
+                    help='after the timed steps, write the (world*32, 200, 6) detections of the last timed step to DIR/detections.npy')
     args = ap.parse_args()
+    if args.steps < 1:
+        ap.error('--steps must be at least 1')
+    if args.dump_outputs and args.impl != 'ours':
+        ap.error('--dump-outputs writes what the CUDA path computed: it needs --impl ours')
     if args.impl == 'reference':
         run_reference(args)
     else:

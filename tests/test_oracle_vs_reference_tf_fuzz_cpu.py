@@ -1,49 +1,15 @@
 """Differential fuzzing of the TensorFlow/Keras half of the oracle against THE REFERENCE'S OWN loss / layer source executed over
 tests/golden/tf_shim.py (see that file for what the stand-in assumes), on random inputs, beyond the fixed vectors of
-tests/golden/ref_tf_shim_golden.npz.  Needs the reference checkout; skipped where it is absent."""
-import os
-import sys
-
+tests/golden/ref_tf_shim_golden.npz.  The inputs are generated here from their seeds; what the reference returned for them is
+stored in tests/golden/ref_fuzz_golden.npz.xz (tests/golden/make_fuzz_golden.py)."""
 import numpy as np
 import pytest
 
-REF = os.environ.get('SSD_REFERENCE_ROOT', '/root/reference')
-pytestmark = pytest.mark.skipif(not os.path.isdir(os.path.join(REF, 'keras_layers')), reason='reference checkout not present')
-HERE = os.path.dirname(os.path.abspath(__file__))
+from test_oracle_vs_reference_fuzz_cpu import check_inputs, ref  # noqa: F401  (ref: the golden fixture)
 
 
-@pytest.fixture(scope='module')
-def ref():
-    np.float = float    # noqa
-    np.int = int        # noqa
-    sys.path.insert(0, REF); sys.path.insert(0, os.path.join(HERE, 'golden'))
-    saved = {k: sys.modules.get(k) for k in ('tensorflow', 'keras', 'keras.backend', 'keras.engine', 'keras.engine.topology',
-                                             'keras.layers', 'keras.models', 'keras.regularizers')}
-    import tf_shim
-    tf_shim.install()
-    try:
-        from keras_layers.keras_layer_DecodeDetections import DecodeDetections
-        from keras_layers.keras_layer_DecodeDetectionsFast import DecodeDetectionsFast
-        from keras_loss_function.keras_ssd_loss import SSDLoss
-        yield dict(DecodeDetections=DecodeDetections, DecodeDetectionsFast=DecodeDetectionsFast, SSDLoss=SSDLoss)
-    finally:
-        for k, v in saved.items():
-            if v is None:
-                sys.modules.pop(k, None)
-            else:
-                sys.modules[k] = v
-        for k in [m for m in sys.modules if m.startswith(('keras_layers', 'keras_loss_function'))]:
-            sys.modules.pop(k, None)
-        sys.path.remove(REF); sys.path.remove(os.path.join(HERE, 'golden'))
-        for alias in ('float', 'int'):
-            if alias in vars(np):
-                delattr(np, alias)
-
-
-@pytest.mark.parametrize('seed', range(20))
-def test_ssd_loss_fuzz(ref, seed):
+def loss_case(seed):
     from oracle import synth
-    from oracle.loss import ssd_loss
     rng = np.random.default_rng(4000 + seed)
     B, P, C = int(rng.integers(1, 4)), int(rng.integers(30, 300)), int(rng.integers(2, 8))
     anchors = rng.uniform(0.1, 0.9, (P, 4))
@@ -58,15 +24,11 @@ def test_ssd_loss_fuzz(ref, seed):
         y_pred[:, :, :C] = 1.0 / C                                             # all losses tie
     y_true[:, :, C:C + 4] = rng.standard_normal((B, P, 4))
     kw = dict(neg_pos_ratio=int(rng.integers(1, 5)), n_neg_min=int(rng.choice([0, 0, 3, 50])), alpha=float(rng.choice([0.5, 1.0, 2.0])))
-    want = np.asarray(ref['SSDLoss'](**kw).compute_loss(y_true.astype(np.float32), y_pred.astype(np.float32)), np.float32)
-    got = ssd_loss(y_true.astype(np.float32), y_pred.astype(np.float32), kw['neg_pos_ratio'], kw['n_neg_min'], kw['alpha'])
-    np.testing.assert_allclose(got, want, rtol=5e-6, atol=1e-6)
+    return y_true.astype(np.float32), y_pred.astype(np.float32), kw
 
 
-@pytest.mark.parametrize('seed', range(20))
-def test_decode_layers_fuzz(ref, seed):
+def decode_layer_case(seed):
     from oracle import synth
-    from oracle.decoder import decode_layer, decode_layer_fast
     rng = np.random.default_rng(5000 + seed)
     P, C, B = int(rng.integers(20, 150)), int(rng.integers(2, 6)), int(rng.integers(1, 3))
     anchors = np.concatenate([rng.uniform(0.1, 0.9, (P, 2)), rng.uniform(0.05, 0.5, (P, 2))], axis=1)
@@ -74,8 +36,26 @@ def test_decode_layers_fuzz(ref, seed):
     kw = dict(confidence_thresh=float(rng.choice([0.01, 0.2, 0.5])), iou_threshold=float(rng.choice([0.3, 0.45, 0.6])),
               top_k=int(rng.choice([3, 20, 200])), nms_max_output_size=int(rng.choice([2, 10, 400])),
               normalize_coords=bool(rng.integers(0, 2)), img_height=120, img_width=160)
-    for cls, fn in ((ref['DecodeDetections'], decode_layer), (ref['DecodeDetectionsFast'], decode_layer_fast)):
-        want = np.asarray(cls(**kw).call(y.astype(np.float32)), np.float32)
+    return y, kw
+
+
+@pytest.mark.parametrize('seed', range(20))
+def test_ssd_loss_fuzz(ref, seed):
+    from oracle.loss import ssd_loss
+    y_true, y_pred, kw = loss_case(seed)
+    check_inputs(ref, 'loss/%d' % seed, kw, y_true, y_pred)
+    want = ref['loss/%d/out' % seed]
+    got = ssd_loss(y_true, y_pred, kw['neg_pos_ratio'], kw['n_neg_min'], kw['alpha'])
+    np.testing.assert_allclose(got, want, rtol=5e-6, atol=1e-6)
+
+
+@pytest.mark.parametrize('seed', range(20))
+def test_decode_layers_fuzz(ref, seed):
+    from oracle.decoder import decode_layer, decode_layer_fast
+    y, kw = decode_layer_case(seed)
+    check_inputs(ref, 'layer/%d' % seed, kw, y)
+    for name, fn in (('DecodeDetections', decode_layer), ('DecodeDetectionsFast', decode_layer_fast)):
+        want = ref['layer/%d/%s' % (seed, name)]
         got = fn(y, kw['confidence_thresh'], kw['iou_threshold'], kw['top_k'], kw['nms_max_output_size'], kw['normalize_coords'], 120, 160)
         assert got.shape == want.shape
         np.testing.assert_array_equal(got[..., :2], want[..., :2])             # class ids and confidences, row by row
