@@ -479,13 +479,15 @@ class SSDModel(KerasTrainingMixin):
         outs = [r.numpy().copy() for r in self.predict_stream(x[i:i + bs] for i in range(0, x.shape[0], bs))]
         return np.concatenate(outs, axis=0)
 
-    def read_layer(self, name, batch):
-        """Activation of a layer after the last forward with this batch size, float32 ndarray (B,h,w,c)."""
+    def read_layer(self, name, batch, training=False):
+        """Activation of a layer after the last forward with this batch size, float32 ndarray (B,h,w,c).  ``training``: of the
+        training plan (``forward_device(..., training=True)``, what ``SSDTrainer`` runs), where a predictor head reads as its
+        raw output, per box [class logits | 4 offsets]."""
         import torch
         i = self.index[name]
         h, w, c = self._shapes[i]
         out = torch.empty((batch, h, w, c), dtype=torch.float32, device='cuda')
-        _ffi.check(_ffi.lib().ssdk_model_read_layer(self._plan(batch)['handle'], i, _ffi.dptr(out), _ffi.stream_ptr()))
+        _ffi.check(_ffi.lib().ssdk_model_read_layer(self._plan(batch, training)['handle'], i, _ffi.dptr(out), _ffi.stream_ptr()))
         return out.cpu().numpy()
 
     def flops(self, batch):
