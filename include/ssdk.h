@@ -165,6 +165,24 @@ typedef struct { int op; int flags; double a0, a1, a2, a3; } ssdk_box_op;
 int ssdk_assemble_batch(ssdk_ctx* ctx, const void* gt_in_dev, int gt_in_f64, const int* offsets_in_dev, int B, int total_in,
                         const ssdk_box_op* ops_dev, int max_ops, float* gt_out_dev, int* offsets_out_dev, int* out_stats_dev,
                         void* stream);
+/* The image half of the same operations, driven by the same lists: B ragged uint8 HWC 3-channel source images (photometric
+ * distortions already applied) -> out_dev (B, out_h, out_w, 3), float32 (out_dtype 0, values 0..255) or uint8 (1).
+ *   src_dev          all images' bytes; image b starts at byte src_offsets_dev[b] (int64) and is src_hw_dev[2b] x src_hw_dev[2b+1]
+ *   CROP_PAD         the CropPad canvas (object_detection_2d_patch_sampling_ops.py:266-313): patch-sized, filled with the
+ *                    background (flags bits 8-15 R, 16-23 G, 24-31 B), the image placed at -patch origin; a patch running past the
+ *                    image is padded with the background too.  SSDExpand = negative origin with background (123, 117, 104).
+ *   FLIP_H / FLIP_V  image[:, ::-1] / image[::-1]; a0 must be the current width / height
+ *   RESIZE           cv2.resize(image, (a3, a2), interpolation=flags bits 8-15): 0 NEAREST, 1 LINEAR, 2 CUBIC, 3 AREA, 4 LANCZOS4
+ *                    (object_detection_2d_geometric_ops.py:61-72); a0 / a1 must be the current size.  Bit-exact to OpenCV's 8-bit
+ *                    arithmetic (CUBIC: to its portable implementation, see DESIGN.md section 4)
+ *   FILTER           no effect on pixels
+ * One fused launch, no intermediate images.  Returns SSDK_ERR_INVALID, before anything is launched, for an empty source image,
+ * a crop/pad parameter that is not an integer or whose origin lies past the image (the reference's ValueError), more than one
+ * RESIZE or a crop/pad / flip after it, a mode outside 0..4, sizes in a FLIP / RESIZE that are not the image's, or a final size
+ * other than (out_h, out_w).  To validate, the call copies the sizes and op lists to the host and synchronises `stream`. */
+int ssdk_assemble_images(ssdk_ctx* ctx, const uint8_t* src_dev, const int64_t* src_offsets_dev, const int* src_hw_dev, int B,
+                         const ssdk_box_op* ops_dev, int max_ops, int out_h, int out_w, int out_dtype /* 0 f32, 1 u8 */, void* out_dev,
+                         void* stream);
 
 /* ------------------------------------------------------------------------------------------
  * Evaluation.  Replaces the per-prediction Python loop of Evaluator.match_predictions

@@ -129,6 +129,8 @@ def lib():
         L.ssdk_eval_cumsum.restype = C.c_int
         L.ssdk_assemble_batch.argtypes = [vp, vp, C.c_int, vp, C.c_int, C.c_int, vp, C.c_int, vp, vp, vp, vp]
         L.ssdk_assemble_batch.restype = C.c_int
+        L.ssdk_assemble_images.argtypes = [vp, vp, vp, vp, C.c_int, vp, C.c_int, C.c_int, C.c_int, C.c_int, vp, vp]
+        L.ssdk_assemble_images.restype = C.c_int
         L.ssdk_l2_normalize.argtypes = [vp, vp, C.c_longlong, C.c_int, vp, vp, vp]
         L.ssdk_l2_normalize.restype = C.c_int
         L.ssdk_conv2d_fwd.argtypes = [vp, vp] + [C.c_int] * 4 + [vp, vp] + [C.c_int] * 11 + [vp, vp]

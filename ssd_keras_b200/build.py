@@ -25,6 +25,7 @@ SOURCES = {
     'decode.cu': ['--fmad=false'],
     'loss.cu': ['--fmad=false'],
     'batch.cu': ['--fmad=false'],
+    'images.cu': ['--fmad=false'],
     'evaluate.cu': ['--fmad=false'],
     'conv.cu': [],
     'model.cu': [],
