@@ -165,8 +165,8 @@ typedef struct { int op; int flags; double a0, a1, a2, a3; } ssdk_box_op;
 int ssdk_assemble_batch(ssdk_ctx* ctx, const void* gt_in_dev, int gt_in_f64, const int* offsets_in_dev, int B, int total_in,
                         const ssdk_box_op* ops_dev, int max_ops, float* gt_out_dev, int* offsets_out_dev, int* out_stats_dev,
                         void* stream);
-/* The image half of the same operations, driven by the same lists: B ragged uint8 HWC 3-channel source images (photometric
- * distortions already applied) -> out_dev (B, out_h, out_w, 3), float32 (out_dtype 0, values 0..255) or uint8 (1).
+/* The image half of the same operations, driven by the same lists: B ragged uint8 HWC 3-channel source images (the output of
+ * ssdk_photometric when the chain distorts them) -> out_dev (B, out_h, out_w, 3), float32 (out_dtype 0, values 0..255) or uint8 (1).
  *   src_dev          all images' bytes; image b starts at byte src_offsets_dev[b] (int64) and is src_hw_dev[2b] x src_hw_dev[2b+1]
  *   CROP_PAD         the CropPad canvas (object_detection_2d_patch_sampling_ops.py:266-313): patch-sized, filled with the
  *                    background (flags bits 8-15 R, 16-23 G, 24-31 B), the image placed at -patch origin; a patch running past the
@@ -183,6 +183,31 @@ int ssdk_assemble_batch(ssdk_ctx* ctx, const void* gt_in_dev, int gt_in_f64, con
 int ssdk_assemble_images(ssdk_ctx* ctx, const uint8_t* src_dev, const int64_t* src_offsets_dev, const int* src_hw_dev, int B,
                          const ssdk_box_op* ops_dev, int max_ops, int out_h, int out_w, int out_dtype /* 0 f32, 1 u8 */, void* out_dev,
                          void* stream);
+/* The photometric distortions that come before SSDExpand in the reference's chains (object_detection_2d_photometric_ops.py),
+ * as a per-image list of pointwise pixel operations on the same ragged uint8 layout ssdk_assemble_images takes.  A pixel is in
+ * uint8 state (the start) or float32 state; the list must end in uint8 state, so the result is ready to be that call's src_dev.
+ *   TO_FLOAT      ConvertDataType('float32')           identity in float32 state
+ *   TO_U8         ConvertDataType('uint8'): np.round (half to even) then astype(uint8); identity in uint8 state
+ *   RGB2HSV       ConvertColor('RGB', 'HSV'): cv2.cvtColor on uint8, OpenCV's 8-bit integer arithmetic       (uint8 state only)
+ *   HSV2RGB       ConvertColor('HSV', 'RGB'): cv2.cvtColor on uint8, bit-exact to OpenCV 4.13's default (AVX2) path: whole
+ *                 32-pixel vectors of a row truncate, the last (width mod 32) pixels round (DESIGN.md section 4) (uint8 state only)
+ *   BRIGHTNESS    Brightness(a0):  clip(x + f32(a0), 0, 255)                                                (float32 state only)
+ *   CONTRAST      Contrast(a0):    clip(127.5 + f32(a0) * (x - 127.5), 0, 255), a0 > 0                     (float32 state only)
+ *   SATURATION    Saturation(a0):  channel 1 = clip(x * f32(a0), 0, 255), a0 > 0                           (float32 state only)
+ *   HUE           Hue(a0):         channel 0 = NumPy's float32 (x + f32(a0)) % 180, a0 in [-180, 180]       (float32 state only)
+ *   CHANNEL_SWAP  ChannelSwap(order): x[..., order], arg = o0 | o1 << 8 | o2 << 16, each in 0..2             (either state)
+ * a0 is the parameter as drawn (a Python float); NumPy 2 rounds it to float32 before combining it with a float32 image, and so
+ * does the kernel.  A list ends at SSDK_PIXOP_END or after max_ops (0..64) entries.  dst_dev may equal src_dev (in place).
+ * One launch.  Returns SSDK_ERR_INVALID, before anything is launched, for an empty image, an unknown operation, a colour
+ * conversion in float32 state, an arithmetic operation in uint8 state, a list that does not end in uint8 state, a NaN
+ * parameter or one the reference's constructors refuse.  To validate, the call copies the sizes and op lists to the host and
+ * synchronises `stream`. */
+typedef enum { SSDK_PIXOP_END = 0, SSDK_PIXOP_TO_FLOAT = 1, SSDK_PIXOP_TO_U8 = 2, SSDK_PIXOP_RGB2HSV = 3, SSDK_PIXOP_HSV2RGB = 4,
+               SSDK_PIXOP_BRIGHTNESS = 5, SSDK_PIXOP_CONTRAST = 6, SSDK_PIXOP_SATURATION = 7, SSDK_PIXOP_HUE = 8,
+               SSDK_PIXOP_CHANNEL_SWAP = 9 } ssdk_pixel_op_kind;
+typedef struct { int op; int arg; double a0; } ssdk_pixel_op;
+int ssdk_photometric(ssdk_ctx* ctx, const uint8_t* src_dev, uint8_t* dst_dev, const int64_t* src_offsets_dev, const int* src_hw_dev,
+                     int B, const ssdk_pixel_op* ops_dev, int max_ops, void* stream);
 
 /* ------------------------------------------------------------------------------------------
  * Evaluation.  Replaces the per-prediction Python loop of Evaluator.match_predictions

@@ -53,6 +53,15 @@ class BoxOp(C.Structure):
 BOXOP_END, BOXOP_CROP_PAD, BOXOP_FLIP_H, BOXOP_FLIP_V, BOXOP_RESIZE, BOXOP_FILTER = range(6)
 
 
+class PixelOp(C.Structure):
+    _fields_ = [('op', C.c_int), ('arg', C.c_int), ('a0', C.c_double)]
+
+
+(PIXOP_END, PIXOP_TO_FLOAT, PIXOP_TO_U8, PIXOP_RGB2HSV, PIXOP_HSV2RGB, PIXOP_BRIGHTNESS, PIXOP_CONTRAST, PIXOP_SATURATION, PIXOP_HUE,
+ PIXOP_CHANNEL_SWAP) = range(10)
+MAX_PIXEL_OPS = 64
+
+
 class LossWsLayout(C.Structure):
     _fields_ = [('bytes', C.c_longlong), ('counts_offset', C.c_longlong), ('counts_n', C.c_longlong), ('hist1_offset', C.c_longlong),
                 ('hist2_offset', C.c_longlong), ('hist_n', C.c_longlong), ('ties_offset', C.c_longlong)]
@@ -131,6 +140,8 @@ def lib():
         L.ssdk_assemble_batch.restype = C.c_int
         L.ssdk_assemble_images.argtypes = [vp, vp, vp, vp, C.c_int, vp, C.c_int, C.c_int, C.c_int, C.c_int, vp, vp]
         L.ssdk_assemble_images.restype = C.c_int
+        L.ssdk_photometric.argtypes = [vp, vp, vp, vp, vp, C.c_int, vp, C.c_int, vp]
+        L.ssdk_photometric.restype = C.c_int
         L.ssdk_l2_normalize.argtypes = [vp, vp, C.c_longlong, C.c_int, vp, vp, vp]
         L.ssdk_l2_normalize.restype = C.c_int
         L.ssdk_conv2d_fwd.argtypes = [vp, vp] + [C.c_int] * 4 + [vp, vp] + [C.c_int] * 11 + [vp, vp]

@@ -26,6 +26,7 @@ SOURCES = {
     'loss.cu': ['--fmad=false'],
     'batch.cu': ['--fmad=false'],
     'images.cu': ['--fmad=false'],
+    'photometric.cu': ['--fmad=false'],
     'evaluate.cu': ['--fmad=false'],
     'conv.cu': [],
     'model.cu': [],

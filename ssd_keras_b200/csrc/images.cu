@@ -396,7 +396,10 @@ extern "C" int ssdk_assemble_images(ssdk_ctx* ctx, const uint8_t* src_dev, const
   const size_t tile = ((size_t)kBandRows * out_w * 3 + 15) / 16 * 16;
   const size_t smem = tile + (size_t)max_ops * sizeof(PixOp);
   SSDK_REQUIRE(smem <= 200 * 1024, "ssdk_assemble_images: output width %d is too large", out_w);
-  if (smem > 48 * 1024) SSDK_CHECK_CUDA(cudaFuncSetAttribute(image_ops_kernel, cudaFuncAttributeMaxDynamicSharedMemorySize, (int)smem));
+  cudaFuncAttributes fa;                                                       // the static shared memory counts towards 48 KB too
+  SSDK_CHECK_CUDA(cudaFuncGetAttributes(&fa, image_ops_kernel));
+  if (smem + fa.sharedSizeBytes > 48 * 1024)
+    SSDK_CHECK_CUDA(cudaFuncSetAttribute(image_ops_kernel, cudaFuncAttributeMaxDynamicSharedMemorySize, (int)smem));
   const int threads = min(512, max(64, (out_w + 31) / 32 * 32));
   const dim3 grid((out_h + kBandRows - 1) / kBandRows, B);
   SSDK_REQUIRE(grid.y <= 65535, "ssdk_assemble_images: batch of %d is too large", B);

@@ -12,8 +12,13 @@ host round trip.
 The image half runs there too: ``assemble_images_device`` uploads the ragged uint8 source images once (one pinned buffer) and
 ``ssdk_assemble_images`` applies the same operation lists to the pixels -- ``CropPad``'s canvas, ``Flip`` and ``cv2.resize`` with
 any of the five modes ``ResizeRandomInterp`` draws from -- in one fused kernel that writes the ``(B, H, W, 3)`` model input.
-``augment_batch_device`` runs both halves from one list per image.  Decoding and photometric distortions stay with the caller:
-they come first in the reference's chain, so the images handed in are what enters ``SSDExpand``."""
+``augment_batch_device`` runs both halves from one list per image.
+
+The photometric distortions, which come first in the reference's chains, run there as well: ``pixel_ops=`` takes one list of
+pointwise pixel operations per image (built with ``convert_data_type`` / ``convert_color`` / ``brightness`` / ``contrast`` /
+``saturation`` / ``hue`` / ``channel_swap``, or drawn like ``SSDPhotometricDistortions`` by ``ssd_photometric_distortions``),
+and ``ssdk_photometric`` applies them to the uploaded sources in place before ``ssdk_assemble_images`` reads them, so canvas
+backgrounds are never distorted.  Decoding stays with the caller."""
 import ctypes as C
 
 import numpy as np
@@ -108,6 +113,151 @@ def encode_batch_device(encoder, labels_list, ops_per_image=None, out=None):
     return encoder.encode_device_offsets(gt, offs, total, max_g, out=out)
 
 
+def convert_data_type(to='uint8'):
+    """``ConvertDataType`` (photometric_ops.py:62-86): ``np.round(x).astype(uint8)`` or ``astype(float32)``."""
+    if not (to == 'uint8' or to == 'float32'):
+        raise ValueError("`to` can be either of 'uint8' or 'float32'.")
+    return (_ffi.PIXOP_TO_U8 if to == 'uint8' else _ffi.PIXOP_TO_FLOAT, 0, 0.0)
+
+
+def convert_color(current='RGB', to='HSV'):
+    """``ConvertColor`` (photometric_ops.py:23-60) between RGB and HSV, i.e. ``cv2.cvtColor`` on a uint8 image.  Grayscale
+    conversions are not supported (``NotImplementedError``); a conversion to the current space is the identity."""
+    if not ((current in {'RGB', 'HSV'}) and (to in {'RGB', 'HSV', 'GRAY'})):
+        raise NotImplementedError
+    if to == 'GRAY':
+        raise NotImplementedError('grayscale conversions are not supported on the device')
+    if current == to:
+        return channel_swap((0, 1, 2))
+    return (_ffi.PIXOP_RGB2HSV if to == 'HSV' else _ffi.PIXOP_HSV2RGB, 0, 0.0)
+
+
+def brightness(delta):
+    """``Brightness`` (photometric_ops.py:225-246) on a float32 RGB image: ``clip(x + delta, 0, 255)``."""
+    delta = float(delta)
+    if delta != delta:
+        raise ValueError('`delta` must not be NaN.')
+    return (_ffi.PIXOP_BRIGHTNESS, 0, delta)
+
+
+def _factor(kind, factor):
+    factor = float(factor)
+    if factor <= 0.0:
+        raise ValueError('It must be `factor > 0`.')
+    if not np.isfinite(factor):
+        raise ValueError('`factor` must be finite.')
+    return (kind, 0, factor)
+
+
+def contrast(factor):
+    """``Contrast`` (photometric_ops.py:281-304) on a float32 RGB image: ``clip(127.5 + factor * (x - 127.5), 0, 255)``."""
+    return _factor(_ffi.PIXOP_CONTRAST, factor)
+
+
+def saturation(factor):
+    """``Saturation`` (photometric_ops.py:166-189) on a float32 HSV image: channel 1 = ``clip(x * factor, 0, 255)``."""
+    return _factor(_ffi.PIXOP_SATURATION, factor)
+
+
+def hue(delta):
+    """``Hue`` (photometric_ops.py:110-133) on a float32 HSV image: channel 0 = ``(x + delta) % 180.0``."""
+    delta = float(delta)
+    if not (-180 <= delta <= 180):
+        raise ValueError("`delta` must be in the closed interval `[-180, 180]`.")
+    return (_ffi.PIXOP_HUE, 0, delta)
+
+
+def channel_swap(order):
+    """``ChannelSwap`` (photometric_ops.py:438-455): ``x[..., order]`` for three indices in 0..2."""
+    order = tuple(int(i) for i in order)
+    if len(order) != 3 or any(i < 0 or i > 2 for i in order):
+        raise ValueError('`order` must be three channel indices in 0..2.')
+    return (_ffi.PIXOP_CHANNEL_SWAP, order[0] | (order[1] << 8) | (order[2] << 16), 0.0)
+
+
+# RandomChannelSwap's permutations (photometric_ops.py:470-472)
+CHANNEL_SWAP_PERMUTATIONS = ((0, 2, 1), (1, 0, 2), (1, 2, 0), (2, 0, 1), (2, 1, 0))
+
+
+def ssd_photometric_distortions():
+    """One image's pixel-op list for ``SSDPhotometricDistortions.__call__`` (data_augmentation_chain_original_ssd.py:146-206),
+    drawn from ``np.random`` with the same calls in the same order: ``choice(2)`` picks the sequence, then every ``Random*`` step
+    draws ``uniform(0, 1)`` and, when it applies, its value.  Afterwards ``np.random`` is in the state the reference's call leaves
+    it in.  The list always holds the uint8 HSV round trip, which the reference runs whether or not a distortion applies."""
+    def maybe(prob, draw):
+        p = np.random.uniform(0, 1)
+        return [draw()] if p >= (1.0 - prob) else []
+
+    def bright():
+        return maybe(0.5, lambda: brightness(np.random.uniform(-32.0, 32.0)))
+
+    def contr():
+        return maybe(0.5, lambda: contrast(np.random.uniform(0.5, 1.5)))
+
+    def hsv_part():
+        return ([convert_data_type('uint8'), convert_color('RGB', 'HSV'), convert_data_type('float32')]
+                + maybe(0.5, lambda: saturation(np.random.uniform(0.5, 1.5)))
+                + maybe(0.5, lambda: hue(np.random.uniform(-18, 18)))
+                + [convert_data_type('uint8'), convert_color('HSV', 'RGB')])
+
+    def swap():
+        return maybe(0.0, lambda: channel_swap(CHANNEL_SWAP_PERMUTATIONS[np.random.randint(5)]))
+
+    if np.random.choice(2):
+        ops = [convert_data_type('float32')] + bright()
+        ops += contr()
+        ops += hsv_part()
+    else:
+        ops = [convert_data_type('float32')] + bright()
+        ops += hsv_part()
+        ops += [convert_data_type('float32')] + contr() + [convert_data_type('uint8')]
+    return ops + swap()
+
+
+def _pixel_state(b, ops):
+    """Check image b's pixel-op list like ``ssdk_photometric`` does; raise ValueError for what it refuses."""
+    if len(ops) > _ffi.MAX_PIXEL_OPS:
+        raise ValueError('image %d: more than %d pixel operations' % (b, _ffi.MAX_PIXEL_OPS))
+    u8 = True
+    for i, o in enumerate(ops):
+        kind, arg, a0 = int(o[0]), int(o[1]), float(o[2])
+        if kind == _ffi.PIXOP_END:
+            break
+        if kind == _ffi.PIXOP_TO_FLOAT:
+            u8 = False
+        elif kind == _ffi.PIXOP_TO_U8:
+            u8 = True
+        elif kind in (_ffi.PIXOP_RGB2HSV, _ffi.PIXOP_HSV2RGB):
+            if not u8:
+                raise ValueError('image %d, op %d: colour conversion of a float32 image (convert it to uint8 first)' % (b, i))
+        elif kind in (_ffi.PIXOP_BRIGHTNESS, _ffi.PIXOP_CONTRAST, _ffi.PIXOP_SATURATION, _ffi.PIXOP_HUE):
+            if u8:
+                raise ValueError('image %d, op %d: photometric arithmetic on a uint8 image (convert it to float32 first)' % (b, i))
+            if a0 != a0:
+                raise ValueError('image %d, op %d: the parameter is NaN' % (b, i))
+            if kind == _ffi.PIXOP_HUE and not -180 <= a0 <= 180:
+                raise ValueError('image %d, op %d: `delta` must be in the closed interval `[-180, 180]`.' % (b, i))
+            if kind in (_ffi.PIXOP_CONTRAST, _ffi.PIXOP_SATURATION) and not (a0 > 0.0 and np.isfinite(a0)):
+                raise ValueError('image %d, op %d: It must be `factor > 0`.' % (b, i))
+        elif kind == _ffi.PIXOP_CHANNEL_SWAP:
+            if arg < 0 or arg >> 24 or any(((arg >> s) & 255) > 2 for s in (0, 8, 16)):
+                raise ValueError('image %d, op %d: channel order %#x has an index outside 0..2' % (b, i, arg))
+        else:
+            raise ValueError('image %d: unknown pixel operation %d' % (b, kind))
+    if not u8:
+        raise ValueError('image %d: the pixel operations end in float32 state (end them with convert_data_type(\'uint8\'))' % b)
+
+
+def _pack_pixel_ops(pixel_ops, B):
+    max_ops = max([len(o) for o in pixel_ops] + [0])
+    arr = (_ffi.PixelOp * max(B * max_ops, 1))()
+    for b, lst in enumerate(pixel_ops):
+        for i, o in enumerate(lst):
+            e = arr[b * max_ops + i]
+            e.op, e.arg, e.a0 = int(o[0]), int(o[1]), float(o[2])
+    return bytes(arr)[:B * max_ops * C.sizeof(_ffi.PixelOp)], max_ops
+
+
 def _image_extents(b, h, w, ops):
     """Walk image b's op list like ``ssdk_assemble_images`` does; raise ValueError for what it refuses.  Returns the final size."""
     resized = False
@@ -159,12 +309,13 @@ def _pack_ops(ops_per_image, B):
     return bytes(arr)[:B * max_ops * C.sizeof(_ffi.BoxOp)], max_ops
 
 
-def assemble_images_device(images, ops_per_image, height, width, dtype=None, out=None):
-    """The image half of the augmentation chain on the device.  ``images``: B uint8 ``(h_i, w_i, 3)`` arrays (the photometric
-    distortions already applied); ``ops_per_image``: B op lists built with ``crop_pad`` / ``flip`` / ``resize`` / ``box_filter``
-    (``box_filter`` does not touch pixels), each ending at ``(height, width)``.  Returns a CUDA tensor ``(B, height, width, 3)``
-    in ``dtype`` (``torch.float32``, the model input, or ``torch.uint8``), written into ``out`` if given.  Validation errors
-    are raised as ValueError before anything is uploaded or launched."""
+def assemble_images_device(images, ops_per_image, height, width, dtype=None, out=None, pixel_ops=None):
+    """The image half of the augmentation chain on the device.  ``images``: B uint8 ``(h_i, w_i, 3)`` arrays;
+    ``ops_per_image``: B op lists built with ``crop_pad`` / ``flip`` / ``resize`` / ``box_filter`` (``box_filter`` does not touch
+    pixels), each ending at ``(height, width)``.  ``pixel_ops``: optional B lists of photometric pixel operations (see
+    ``ssd_photometric_distortions``), applied to the sources before the geometric operations, in one extra launch.  Returns a
+    CUDA tensor ``(B, height, width, 3)`` in ``dtype`` (``torch.float32``, the model input, or ``torch.uint8``), written into
+    ``out`` if given.  Validation errors are raised as ValueError before anything is uploaded or launched."""
     import torch
     dtype = torch.float32 if dtype is None else dtype
     if dtype not in (torch.float32, torch.uint8):
@@ -191,6 +342,11 @@ def assemble_images_device(images, ops_per_image, height, width, dtype=None, out
         hw = _image_extents(b, a.shape[0], a.shape[1], ops_per_image[b] if ops_per_image is not None else [])
         if hw != (height, width):
             raise ValueError('image %d ends at %d x %d, the batch is %d x %d' % (b, hw[0], hw[1], height, width))
+    if pixel_ops is not None:
+        if len(pixel_ops) != B:
+            raise ValueError('pixel_ops must have one list per batch item')
+        for b, lst in enumerate(pixel_ops):
+            _pixel_state(b, lst)
     if out is not None and (not out.is_cuda or out.dtype != dtype or tuple(out.shape) != (B, height, width, 3) or not out.is_contiguous()):
         raise ValueError('out must be a contiguous CUDA tensor (%d, %d, %d, 3) of %s' % (B, height, width, dtype))
     ops_bytes, max_ops = _pack_ops(ops_per_image, B)
@@ -202,6 +358,10 @@ def assemble_images_device(images, ops_per_image, height, width, dtype=None, out
     o_hw = o_offs + al(offs.nbytes)
     o_pix = o_hw + al(hw.nbytes)
     total = o_pix + int(sum(a.size for a in arrs))
+    if pixel_ops is not None:                                                                   # [... | pixels | pixel ops]
+        px_bytes, px_max_ops = _pack_pixel_ops(pixel_ops, B)
+        o_px_ops = al(total)
+        total = o_px_ops + len(px_bytes)
     host = torch.empty((total,), dtype=torch.uint8, pin_memory=True)
     hv = host.numpy()
     hv[:len(ops_bytes)] = np.frombuffer(ops_bytes, np.uint8)
@@ -211,19 +371,26 @@ def assemble_images_device(images, ops_per_image, height, width, dtype=None, out
     for a in arrs:
         hv[pos:pos + a.size] = a.reshape(-1)
         pos += a.size
+    if pixel_ops is not None:
+        hv[o_px_ops:o_px_ops + len(px_bytes)] = np.frombuffer(px_bytes, np.uint8)
     dev = host.cuda(non_blocking=True)
     base = dev.data_ptr()
     if out is None:
         out = torch.empty((B, height, width, 3), dtype=dtype, device='cuda')
+    if pixel_ops is not None:                                                  # in place on this call's own copy of the sources
+        _ffi.check(_ffi.lib().ssdk_photometric(_ffi.context(), C.c_void_p(base + o_pix), C.c_void_p(base + o_pix), C.c_void_p(base + o_offs),
+                                               C.c_void_p(base + o_hw), B, C.c_void_p(base + o_px_ops) if px_max_ops else C.c_void_p(0),
+                                               int(px_max_ops), _ffi.stream_ptr()))
     _ffi.check(_ffi.lib().ssdk_assemble_images(_ffi.context(), C.c_void_p(base + o_pix), C.c_void_p(base + o_offs), C.c_void_p(base + o_hw), B,
                                                C.c_void_p(base + 0) if max_ops else C.c_void_p(0), int(max_ops), height, width,
                                                0 if dtype == torch.float32 else 1, _ffi.dptr(out), _ffi.stream_ptr()))
     return out
 
 
-def augment_batch_device(images, labels_list, ops_per_image, height, width):
-    """The geometric half of ``SSDDataAugmentation`` for a batch, pixels and boxes from ONE op list per image: returns
-    ``(images (B, height, width, 3) float32, (gt_dev, offsets_dev, stats_dev, total_upper, max_upper))``, the second part being
-    what ``assemble_batch_device`` returns (feed it to ``SSDInputEncoder.encode_device_offsets``)."""
-    imgs = assemble_images_device(images, ops_per_image, height, width)
+def augment_batch_device(images, labels_list, ops_per_image, height, width, pixel_ops=None):
+    """``SSDDataAugmentation`` for a batch, pixels and boxes from ONE op list per image (plus, optionally, one photometric
+    ``pixel_ops`` list per image, which only touches pixels): returns ``(images (B, height, width, 3) float32, (gt_dev,
+    offsets_dev, stats_dev, total_upper, max_upper))``, the second part being what ``assemble_batch_device`` returns (feed it to
+    ``SSDInputEncoder.encode_device_offsets``)."""
+    imgs = assemble_images_device(images, ops_per_image, height, width, pixel_ops=pixel_ops)
     return imgs, assemble_batch_device(labels_list, ops_per_image)

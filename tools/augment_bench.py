@@ -9,7 +9,13 @@ B*300*300*3*4 written) and their rate as a fraction of the B200 data-sheet HBM b
 same chain is also timed on the host (NumPy canvas + cv2.resize, one image after another) and the host's core count is stated.
 The card's name and power limit are read in the same run.
 
-    python tools/augment_bench.py [--iters 200] [--warmup 20] [--out FILE.json]
+--photometric adds a ``photometric`` object to the result: the same sources with one seeded ``ssd_photometric_distortions()``
+list per image (np.random.seed(2024)), timed as the ssdk_photometric pass alone (sources -> a second buffer) and as the whole
+chain (ssdk_photometric in place, then ssdk_assemble_images), with the pass's algorithmic bytes (2 x source bytes: read once,
+written once) as a fraction of 7.7 TB/s; and, when cv2 is importable, the host equivalent (NumPy float32 ops + cv2.cvtColor, one
+image after another).
+
+    python tools/augment_bench.py [--iters 200] [--warmup 20] [--photometric] [--out FILE.json]
 """
 import argparse
 import json
@@ -62,6 +68,52 @@ def host_chain(images, plain):
     return out
 
 
+def host_photometric(images, pixel_ops):
+    """SSDPhotometricDistortions' arithmetic on the host, one image after another: NumPy float32 ops and cv2.cvtColor."""
+    import cv2
+    from ssd_keras_b200 import _ffi as F
+    out = []
+    for img, ops in zip(images, pixel_ops):
+        x = img
+        for kind, arg, a0 in ops:
+            if kind == F.PIXOP_TO_FLOAT:
+                x = x.astype(np.float32)
+            elif kind == F.PIXOP_TO_U8:
+                x = np.round(x, decimals=0).astype(np.uint8)
+            elif kind == F.PIXOP_RGB2HSV:
+                x = cv2.cvtColor(x, cv2.COLOR_RGB2HSV)
+            elif kind == F.PIXOP_HSV2RGB:
+                x = cv2.cvtColor(x, cv2.COLOR_HSV2RGB)
+            elif kind == F.PIXOP_BRIGHTNESS:
+                x = np.clip(x + a0, 0, 255)
+            elif kind == F.PIXOP_CONTRAST:
+                x = np.clip(127.5 + a0 * (x - 127.5), 0, 255)
+            elif kind == F.PIXOP_SATURATION:
+                x[:, :, 1] = np.clip(x[:, :, 1] * a0, 0, 255)
+            elif kind == F.PIXOP_HUE:
+                x[:, :, 0] = (x[:, :, 0] + a0) % 180.0
+            else:
+                x = x[:, :, [arg & 255, (arg >> 8) & 255, (arg >> 16) & 255]]
+        out.append(x)
+    return out
+
+
+def time_us(fn, iters, warmup):
+    import torch
+    for _ in range(warmup):
+        fn()
+    torch.cuda.synchronize()
+    times = []
+    for _ in range(iters):
+        e0, e1 = torch.cuda.Event(enable_timing=True), torch.cuda.Event(enable_timing=True)
+        e0.record()
+        fn()
+        e1.record()
+        e1.synchronize()
+        times.append(e0.elapsed_time(e1) * 1e3)
+    return times
+
+
 def gpu_info():
     try:
         r = subprocess.run(['nvidia-smi', '--query-gpu=name,power.limit,clocks.max.sm', '--format=csv,noheader'], capture_output=True,
@@ -75,6 +127,7 @@ def main():
     ap = argparse.ArgumentParser()
     ap.add_argument('--iters', type=int, default=200)
     ap.add_argument('--warmup', type=int, default=20)
+    ap.add_argument('--photometric', action='store_true')
     ap.add_argument('--out', default=None)
     args = ap.parse_args()
     import torch
@@ -134,11 +187,76 @@ def main():
         res['host_max_abs_diff'] = int(np.abs(ref - out.cpu().numpy()).max())
     except ImportError:
         res['host_cv2_us_per_batch'] = None
+    if args.photometric:
+        res['photometric'] = photometric_rows(args, images, ops, src, offs, hw, ops_dev, max_ops, out2)
     line = json.dumps(res)
     print(line)
     if args.out:
         with open(args.out, 'w') as f:
             f.write(line + '\n')
+
+
+def photometric_rows(args, images, ops, src, offs, hw, ops_dev, max_ops, out2):
+    import torch
+    from oracle import photometric
+    from ssd_keras_b200 import _ffi
+    from ssd_keras_b200.data_generator import batch_assembly as ba
+    np.random.seed(2024)
+    px = [ba.ssd_photometric_distortions() for _ in range(B)]
+    raw, px_max = ba._pack_pixel_ops(px, B)
+    px_dev = torch.frombuffer(bytearray(raw), dtype=torch.uint8).cuda()
+    dst = torch.empty_like(src)
+    work = torch.empty_like(src)
+    L, ctx = _ffi.lib(), _ffi.context()
+
+    def alone():
+        _ffi.check(L.ssdk_photometric(ctx, _ffi.dptr(src), _ffi.dptr(dst), _ffi.dptr(offs), _ffi.dptr(hw), B, _ffi.dptr(px_dev), px_max,
+                                      _ffi.stream_ptr()))
+
+    def whole():
+        work.copy_(src)                                                    # the in-place pass needs fresh sources each time
+        _ffi.check(L.ssdk_photometric(ctx, _ffi.dptr(work), _ffi.dptr(work), _ffi.dptr(offs), _ffi.dptr(hw), B, _ffi.dptr(px_dev), px_max,
+                                      _ffi.stream_ptr()))
+        _ffi.check(L.ssdk_assemble_images(ctx, _ffi.dptr(work), _ffi.dptr(offs), _ffi.dptr(hw), B, _ffi.dptr(ops_dev), max_ops, OUT, OUT, 0,
+                                          _ffi.dptr(out2), _ffi.stream_ptr()))
+
+    def copy_only():
+        work.copy_(src)
+
+    t_alone = time_us(alone, args.iters, args.warmup)
+    t_whole = time_us(whole, args.iters, args.warmup)
+    t_copy = time_us(copy_only, args.iters, args.warmup)
+    want = photometric.apply_images(images, px)
+    got = dst.cpu().numpy()
+    pos = 0
+    for w in want:
+        assert np.array_equal(got[pos:pos + w.size], w.reshape(-1))
+        pos += w.size
+    src_bytes = int(sum(a.size for a in images))
+    med = float(np.median(t_alone))
+    r = {'pass_median_us': round(med, 2), 'pass_p10_us': round(float(np.percentile(t_alone, 10)), 2),
+         'pass_p90_us': round(float(np.percentile(t_alone, 90)), 2), 'pass_algorithmic_bytes': 2 * src_bytes,
+         'pass_achieved_GBps': round(2 * src_bytes / (med * 1e-6) / 1e9, 1),
+         'pass_hbm_fraction': round(2 * src_bytes / (med * 1e-6) / HBM_BYTES_PER_S, 4),
+         'chain_median_us': round(float(np.median(t_whole)) - float(np.median(t_copy)), 2),
+         'chain_note': 'photometric in place + assemble_images, minus the median of the source copy each timed call makes',
+         'source_copy_median_us': round(float(np.median(t_copy)), 2), 'pixel_ops_per_image': [len(p) for p in px]}
+    try:
+        import cv2
+        host_photometric(images, px)
+        t = []
+        for _ in range(5):
+            t0 = time.perf_counter()
+            h = host_photometric(images, px)
+            t.append((time.perf_counter() - t0) * 1e6)
+        r['host_us_per_batch'] = round(float(np.median(t)), 1)
+        r['host_cores'] = os.cpu_count()
+        r['host_cv2_threads'] = cv2.getNumThreads()
+        r['host_cv2_version'] = cv2.__version__
+        r['host_max_abs_diff'] = int(max(np.abs(a.astype(int) - b.astype(int)).max() for a, b in zip(h, want)))
+    except ImportError:
+        r['host_us_per_batch'] = None
+    return r
 
 
 if __name__ == '__main__':
